@@ -26,6 +26,10 @@ reused inside the timed region), and one step's input is far larger than the 126
 `--impl reference` times the reference's own CPU md_script_eval_frame_range (oracle/_ref/ref_harness_fast: the unmodified mdlib
 sources compiled with their shipped -O3 -ffast-math flags) on all host cores for the same script/workload: ONE process, frames already in
 memory, untimed warm-up passes inside it, every step a bounded sample of 8 frames per thread.
+
+`--dump-outputs DIR` writes, after the timed steps, the values array of every result property of the config as DIR/<name>.npy (float32):
+what a caller of the timed path receives after its last step (rdf: 1024 bin values + 1024 weights; sdf: the 128^3 volume). The frames are
+generated from fixed seeds, so runs with the same arguments see the same inputs and two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -39,6 +43,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: nothing is written there, byte-code caches included
 
 UNIT = "frames/s"
 WATER_N, WATER_SEED = 32, 1234
@@ -313,11 +318,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-iso", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None)
     # rehearsal switches for the N>1 flow on a ONE-GPU machine (never set by the driver): every rank on cuda:0 and gloo instead of NCCL, which refuses
     # two ranks on one device. Everything else — torchrun environment, sharding, barriers, the exchange step, max over ranks, rank-0 line — is the real flow.
     ap.add_argument("--dist-backend", default="nccl", choices=["nccl", "gloo"])
     ap.add_argument("--one-device", action="store_true")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         return impl_reference(args, cfg)
@@ -396,6 +404,9 @@ def main():
     for name in cfg["results"]:
         d = plan.property_data(name)
         checks[name + "_sum_per_frame"] = float(np.float64(d.values[:1024] if d.weights is not None else d.values).sum())
+        if args.dump_outputs and rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), d.values.astype(np.float32))
 
     # ---- end-to-end through the host API: pinned host frames -> (gather of the atoms the script reads) -> H2D -> kernels -> D2H of the step's results
     e2e = None

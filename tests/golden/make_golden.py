@@ -39,6 +39,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import refio  # noqa: E402
 
 HARNESS = os.path.join(ROOT, "oracle", "_ref", "ref_harness_strict")
+SHIM = os.path.join(ROOT, "oracle", "_ref", "shim_harness")
 SYNTH = os.path.join(ROOT, "oracle", "build", "synth_tool")
 
 
@@ -290,6 +291,8 @@ def water32_full(tmp):
     out = dict(script=np.array(script), n=np.int32(n), seed=np.int32(seed), cells=cells, cell_flags=flags,
                frames_sha256=np.array([hashlib.sha256(np.ascontiguousarray(f).tobytes()).hexdigest() for f in frames]))
     pack(out, refio.read_refout(o), list(range(F)))
+    for k in [k for k in out if k.startswith("v__") and k.endswith("_idx")]:   # voxel index lists -> bit mask of the non-zero voxels: half the size
+        mask = np.zeros(128 ** 3, bool); mask[out.pop(k)] = True; out[k[:-4] + "_mask"] = np.packbits(mask)   # compressed (helpers.dense_from_mask)
     np.savez_compressed(os.path.join(HERE, "water32_full.npz"), **out)
 
 
@@ -334,6 +337,32 @@ def dyn6(tmp):
         sub = {}; pack(sub, refio.read_refout(o), list(range(F)))
         for k, v in sub.items(): out[f"{tag}_{k}"] = v
     np.savez_compressed(os.path.join(HERE, "dyn6.npz"), **out)
+
+
+def forms45(tmp):
+    """The 45 statement forms of tests/test_emulated_library.py (PROBE_FORMS, one script) on the first 2 frames of water6 (w) and tric6 (t), each
+    box's topology from the generator seed stored with it: per-frame bins / voxels and full values of every property, as pack() stores them."""
+    from test_emulated_library import PROBE_FORMS
+    script = " ".join(PROBE_FORMS); out = {"script": np.array(script)}; F = 2
+    for tag, name, seed in (("w", "water6.npz", 77), ("t", "tric6.npz", 91)):
+        g = np.load(os.path.join(HERE, name))
+        gro, raw, o = os.path.join(tmp, tag + "f.gro"), os.path.join(tmp, tag + "f.raw"), os.path.join(tmp, tag + "f.out")
+        run(SYNTH, "water-gro", "6", str(seed), gro); refio.write_raw_traj(raw, g["frames"][:F], g["cells"][:F], g["cell_flags"][:F])
+        run(HARNESS, "eval", "--sys", gro, "--traj", f"raw:{raw}", "--script", script, "--out", o, "--perframe", f"0:{F}", "--full", f"0:{F}")
+        sub = {}; pack(sub, refio.read_refout(o), list(range(F)))
+        out.update({f"{tag}_{k}": v for k, v in sub.items()}); out[f"{tag}_seed"] = np.int32(seed)
+    np.savez_compressed(os.path.join(HERE, "forms45.npz"), **out)
+
+
+def shim_lowered(tmp):
+    """integration/md_script_mdgpu.inl's lowering of a compiled md_script IR (oracle/_ref/shim_harness `lower`, the reference's own front-end) for the
+    scripts of tests/test_integration_shim.py on the water6 topology (seed 77): the MDLOWER3 byte stream as written."""
+    from test_integration_shim import SCRIPT, SCRIPT_NEW
+    script = SCRIPT + " " + SCRIPT_NEW
+    gro, o = os.path.join(tmp, "sl.gro"), os.path.join(tmp, "sl.bin")
+    run(SYNTH, "water-gro", "6", "77", gro)
+    run(SHIM, "lower", "--sys", gro, "--script", script, "--out", o)
+    np.savez_compressed(os.path.join(HERE, "shim_lowered.npz"), script=np.array(script), lowered=np.fromfile(o, np.uint8))
 
 
 def backbone(tmp):
@@ -398,7 +427,8 @@ if __name__ == "__main__":
     subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "oracle"])
     only = sys.argv[1:]   # e.g. `python make_golden.py water32_full water12_avg` regenerates just those
     gens = dict(water6=water6, ala50=ala50, membrane6=membrane6, tric6=tric6, tric6_rmsd=tric6_rmsd, pairs6=pairs6, shapes=shapes, xtc_cases=xtc_cases,
-                water32_full=water32_full, water12_avg=water12_avg, backbone=backbone, dyn6=dyn6, arrargs=arrargs, bigcut6=bigcut6, rdftrg6=rdftrg6)
+                water32_full=water32_full, water12_avg=water12_avg, backbone=backbone, dyn6=dyn6, arrargs=arrargs, bigcut6=bigcut6, rdftrg6=rdftrg6,
+                forms45=forms45, shim_lowered=shim_lowered)
     with tempfile.TemporaryDirectory() as tmp:
         for name, fn in gens.items():
             if not only or name in only: fn(tmp)

@@ -22,6 +22,11 @@ def dense_from_sparse(idx, val, n=128 ** 3):
     v = np.zeros(n, np.float32); v[idx] = val; return v
 
 
+def dense_from_mask(mask, val, n=128 ** 3):
+    """volume stored as the np.packbits mask of its non-zero voxels + their values in index order"""
+    v = np.zeros(n, np.float32); v[np.unpackbits(mask, count=n).astype(bool)] = val; return v
+
+
 def golden_system(g):
     """(mass, z, names, comp_off, conn_off, conn_idx) -> selections by element"""
     z = g["z"].astype(int)

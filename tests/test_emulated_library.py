@@ -244,7 +244,7 @@ def test_rdf_kernel_variants_under_emulation(emulated_library):
         plan.close()
 
 
-PROBE_FORMS = [   # statement forms compared with the UNMODIFIED reference evaluated here (oracle/_ref/ref_harness_strict): the sweep that found the silently
+PROBE_FORMS = [   # statement forms compared with the UNMODIFIED reference's results (tests/golden/forms45.npz): the sweep that found the silently
     # flattened rdf target, the missing triclinic min-image of dihedral and the context-relative selections
     "p01 = rdf(residue(1:30), element('O'), 1.0:7.0);", "p02 = rdf(atom(1), atom(2:648), 8.0);", "p03 = rdf(element('H'), element('H'), 5.5);",
     "p04 = sdf(residue(1:30), within(5.0, residue(1:3)), 4.0);", "p05 = density_x(element('O'));", "p06 = density_y(within(6.0, residue(1:5)));",
@@ -265,42 +265,35 @@ PROBE_FORMS = [   # statement forms compared with the UNMODIFIED reference evalu
 
 
 @pytest.mark.parametrize("golden,seed", [("water6.npz", "77"), ("tric6.npz", "91")])
-def test_statement_forms_against_the_reference_itself(emulated_library, tmp_path, golden, seed):
-    """45 statement forms in ONE script: the unmodified reference (oracle/_ref/ref_harness_strict, built from /root/reference) evaluates 2 frames of
-    the golden box here, the library (emulated build) evaluates the Python mirror's lowering of the same statements; distributions and volumes
-    must agree count for count, temporals within 1e-5 (bit-equal for distances). Orthorhombic and changing triclinic cell."""
-    run_statement_forms(tmp_path, golden, seed)
+def test_statement_forms_against_the_reference_itself(emulated_library, golden, seed):
+    """45 statement forms in ONE script: the unmodified reference's evaluation of 2 frames of the golden box (tests/golden/forms45.npz, made by
+    tests/golden/make_golden.py) against the library (emulated build) evaluating the Python mirror's lowering of the same statements; distributions
+    and volumes must agree count for count, temporals within 1e-5 (bit-equal for distances). Orthorhombic and changing triclinic cell."""
+    run_statement_forms(golden, seed)
 
 
-def run_statement_forms(tmp_path, golden, seed):
-    """(also called by tests/test_zz_gpu_new_ops.py with the real library on the device: the harness binary travels, /root/reference is not read)"""
-    import subprocess
+def run_statement_forms(golden, seed):
+    """(also called by tests/test_zz_gpu_new_ops.py with the real library on the device)"""
     import numpy as np
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    harness = os.path.join(root, "oracle", "_ref", "ref_harness_strict"); synth = os.path.join(root, "oracle", "build", "synth_tool")
-    if not os.path.exists(harness): pytest.skip("oracle/_ref/ref_harness_strict not built (needs /root/reference: make -C oracle ref)")
-    sys.path.insert(0, os.path.join(root, "tests", "golden"))
     import refio
     import viamd_b200 as vb
-    from helpers import load_golden, golden_system, vb_system, vb_cell
+    from helpers import load_golden, golden_system, vb_system, vb_cell, dense_from_sparse
     g = load_golden(golden); sysm = vb_system(golden_system(g)); F = 2; script = " ".join(PROBE_FORMS)
-    gro, raw, out = str(tmp_path / "w.gro"), str(tmp_path / "w.raw"), str(tmp_path / "w.out")
-    subprocess.check_call([synth, "water-gro", "6", seed, gro], stdout=subprocess.DEVNULL)
-    refio.write_raw_traj(raw, g["frames"][:F], g["cells"][:F], g["cell_flags"][:F])
-    subprocess.check_call([harness, "eval", "--sys", gro, "--traj", f"raw:{raw}", "--script", script, "--out", out, "--perframe", f"0:{F}", "--full", f"0:{F}"], stdout=subprocess.DEVNULL)
-    ref = refio.read_refout(out)
+    ref = load_golden("forms45.npz"); tag = golden[0]   # w(ater6) / t(ric6)
+    assert str(ref["script"]) == script and int(ref[f"{tag}_seed"]) == int(seed), "forms45.npz is stale: regenerate it with make_golden.py forms45"
     props = vb.compile_script(script, sysm)
     plan = vb.Plan(sysm, props, F, keep_frame_results=True); cells = [vb_cell(g["cells"][f], g["cell_flags"][f]) for f in range(F)]
     plan.set_initial_frame(*g["frames"][0], cells[0]); plan.eval_host_frames(g["frames"][:F], cells, 0)
     for p in props:
-        r = ref[p.name]; d = plan.property_data(p.name)
-        if r.flags & refio.FLAG_VOLUME:
-            assert np.array_equal(plan.counts(p.name).astype(np.float32), sum(r.perframe[f] for f in range(F))), p.name
-        elif r.flags & refio.FLAG_TEMPORAL:
-            a, b = np.asarray(d.values).ravel(), np.asarray(r.full).ravel()
+        k = f"{tag}_{p.name}"; flags = int(ref[k + "__flags"]); d = plan.property_data(p.name)
+        if flags & refio.FLAG_VOLUME:
+            want = sum(dense_from_sparse(ref[f"{k}__pf{f}_idx"], ref[f"{k}__pf{f}_val"]) for f in range(F))
+            assert np.array_equal(plan.counts(p.name).astype(np.float32), want), p.name
+        elif flags & refio.FLAG_TEMPORAL:
+            a, b = np.asarray(d.values).ravel(), ref[k + "__full"].ravel()
             assert a.shape == b.shape and np.allclose(a, b, rtol=1e-5, atol=1e-6), (p.name, a[:4], b[:4])
         elif p.op == vb.OP_RDF:
-            for f in range(F): assert np.array_equal(plan.frame_counts(p.name, f)[0].astype(np.float32), r.perframe[f][:1024]), (p.name, f)
+            for f in range(F): assert np.array_equal(plan.frame_counts(p.name, f)[0].astype(np.float32), ref[k + "__pf"][f, :1024]), (p.name, f)
         else:
-            assert np.allclose(d.values[:1024], r.full[:1024], rtol=1e-5, atol=1e-3), p.name
+            assert np.allclose(d.values[:1024], ref[k + "__full"][:1024], rtol=1e-5, atol=1e-3), p.name
     plan.close()

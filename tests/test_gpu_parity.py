@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 
 import oracle_lib as O
-from helpers import load_golden, cell_from_row, dense_from_sparse, golden_system, sel_element, vb_system, vb_cell
+from helpers import load_golden, cell_from_row, dense_from_mask, dense_from_sparse, golden_system, sel_element, vb_system, vb_cell
 
 pytestmark = pytest.mark.gpu
 RTOL = 1e-5   # north_star: "within 1e-5 relative for float densities"
@@ -393,12 +393,12 @@ def test_full_size_config2_config3_vs_reference_golden_voxel_for_voxel():
         bins, tot = plan.frame_counts("r", f)
         assert np.array_equal(bins.astype(np.float32), g["r__pf"][f, :1024]) and tot == int(g["r__pf"][f, :1024].sum())
         assert np.array_equal(plan.property_data("r").weights, g["r__pf"][f, 1024:])
-        ref = dense_from_sparse(g[f"v__pf{f}_idx"], g[f"v__pf{f}_val"])
+        ref = dense_from_mask(g[f"v__pf{f}_mask"], g[f"v__pf{f}_val"])
         vox = plan.counts("v")
         assert int(vox.sum()) == int(ref.sum()) > 2.5e5 and np.array_equal(vox.astype(np.float32), ref), f"sdf frame {f}"
     plan.clear(); plan.eval_host_frames(frames, cell, 0)
     np.testing.assert_allclose(plan.property_data("r").values[:1024], g["r__full"][:1024], rtol=RTOL, atol=0)
-    np.testing.assert_allclose(plan.property_data("v").values, dense_from_sparse(g["v__full_idx"], g["v__full_val"]), rtol=RTOL, atol=0)
+    np.testing.assert_allclose(plan.property_data("v").values, dense_from_mask(g["v__full_mask"], g["v__full_val"]), rtol=RTOL, atol=0)
     plan.close()
 
 

@@ -1,6 +1,7 @@
 """The drop-in boundary, end to end: the reference's own md_script.c + integration/md_script_mdgpu.inl compiled as one translation
-unit (oracle/_ref/shim_harness, built where /root/reference exists; the prebuilt binary travels to the GPU box).
- - CPU: the shim's lowering of a compiled md_script IR equals viamd_b200.script's lowering (same ops, index lists, cutoffs).
+unit (oracle/_ref/shim_harness, which `make -C oracle ref` builds where the reference sources are present; the tests that run it skip elsewhere).
+ - CPU: the shim's lowering of a compiled md_script IR, stored in tests/golden/shim_lowered.npz, equals viamd_b200.script's lowering (same ops,
+   index lists, cutoffs).
  - GPU: md_script_eval_frame_range (reference CPU path) vs md_script_gpu_eval_frame_range (libmdgpu) on the same script."""
 import json
 import os
@@ -45,12 +46,12 @@ SCRIPT_SHIM_ONLY = ("xr = distance(residue(1), 2) in residue(2:4); ya = distance
 
 def _need():
     if not os.path.exists(SHIM):
-        pytest.skip("oracle/_ref/shim_harness not built (needs /root/reference: make -C oracle ref)")
+        pytest.skip("oracle/_ref/shim_harness not built (needs the reference sources: make -C oracle ref)")
     subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "oracle"])
 
 
-def _read_lowered(path):
-    b = open(path, "rb").read(); assert b[:8] == b"MDLOWER3"
+def _read_lowered(b):
+    assert b[:8] == b"MDLOWER3"
     n, = struct.unpack_from("<Q", b, 8); off = 16; out = []
     for _ in range(n):
         name = b[off:off + 64].split(b"\0")[0].decode(); off += 64
@@ -77,14 +78,14 @@ def _read_lowered(path):
     return out
 
 
-def test_shim_lowering_matches_python_lowering(tmp_path):
-    _need()
+def test_shim_lowering_matches_python_lowering():
+    """The shim's lowering of the md_script IR (stored in tests/golden/shim_lowered.npz by tests/golden/make_golden.py, which runs
+    oracle/_ref/shim_harness `lower` on the water6 topology) equals viamd_b200.script's lowering of the same script."""
     import viamd_b200 as vb
-    gro = str(tmp_path / "w6.gro"); out = str(tmp_path / "low.bin")
-    subprocess.check_call([TOOL, "water-gro", "6", "77", gro])
-    script = SCRIPT + " " + SCRIPT_NEW
-    subprocess.check_call([SHIM, "lower", "--sys", gro, "--script", script, "--out", out], stdout=subprocess.DEVNULL)
-    low = _read_lowered(out)
+    from helpers import load_golden
+    g = load_golden("shim_lowered.npz"); script = SCRIPT + " " + SCRIPT_NEW
+    assert str(g["script"]) == script, "shim_lowered.npz is stale: regenerate it with make_golden.py shim_lowered"
+    low = _read_lowered(g["lowered"].tobytes())
     props = vb.compile_script(script, vb.water_system(6))
     assert [p["name"] for p in low] == [p.name for p in props]
     for a, b in zip(low, props):

@@ -560,8 +560,8 @@ def test_array_and_context_forms_with_empty_or_single_atom_groups():
 
 
 @pytest.mark.parametrize("golden,seed", [("water6.npz", "77"), ("tric6.npz", "91")])
-def test_statement_forms_against_the_reference_itself(tmp_path, golden, seed):
-    """The 45-form sweep of tests/test_emulated_library.py with libmdgpu itself on the device: the prebuilt reference harness (oracle/_ref, no access to
-    /root/reference at run time) evaluates the script on the box's CPU, the library evaluates the lowered statements on the GPU."""
+def test_statement_forms_against_the_reference_itself(golden, seed):
+    """The 45-form sweep of tests/test_emulated_library.py with libmdgpu itself on the device: the library evaluates the lowered statements on the
+    GPU, against the reference's results stored in tests/golden/forms45.npz."""
     from test_emulated_library import run_statement_forms
-    run_statement_forms(tmp_path, golden, seed)
+    run_statement_forms(golden, seed)
